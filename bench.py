@@ -2,6 +2,7 @@
 """bench.py -- transitions/sec through PPO ``Algorithm.update()`` (v1: ``learn()``), obs=17.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c5] [--scaling weak|strong]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY.md 8d): synthetic HalfCheetah-shaped rollout of
 4096 envs x 128 steps per GPU (N = 524,288 transitions, obs 17, act 6), actor/critic MLP[64,64]
@@ -28,6 +29,8 @@ checks itself: ``multi_gpu_check`` = {replicas_equal, loss_rel_err (N ranks vs 1
 ``--config c5`` = BASELINE configs[4] (8192 envs x 256 steps, minibatch N/8); the default run reports it as the extra
 key ``config4`` (strong-scaled over the N GPUs).  The timed arms use the DEFAULT public API (reference-exact
 ``np.random.permutation`` minibatch order); the opt-in device-generated order is reported as ``*_device_order``.
+``--dump-outputs DIR`` writes what the last timed step of the headline arm computed (see ``dump_outputs``): the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -52,6 +55,8 @@ BATCH_SIZE, REPEAT = 16384, 10
 FLOP_TRAIN_PER_ROW = 60_544          # fwd+bwd of actor and critic (SURVEY 8d)
 FLOP_PER_TRANSITION = REPEAT * 81_536 + 11_136
 METRIC = "transitions/sec through Algorithm.learn() (PPO, obs=17)"
+DUMP_ROWS = 1 << 20                  # per-transition outputs of longer rollouts are dumped as a fixed seeded sample of rows
+DUMP_BYTES = 64 << 20
 
 
 def load_peaks() -> tuple[dict, str]:
@@ -210,7 +215,7 @@ def run_reference_arm(args) -> None:
         return
     cfg = CONFIGS[args.config]
     E = int(os.environ.get("TS_BENCH_CPU_ENVS", "1024"))      # 1/4 of configs[1]: 8 minibatches of 16384 per pass
-    res = cpu_reference_run(E, cfg["T"], max(3, args.steps), max(1, min(args.warmup, 1)))
+    res = cpu_reference_run(E, cfg["T"], args.steps, max(1, min(args.warmup, 1)))
     line = {
         "impl": "reference", "metric": METRIC, "value": res["value"], "unit": "transitions/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": res["ms_per_step"], "higher_is_better": True,
@@ -243,11 +248,48 @@ def workload_config(n_gpus: int, config: str = "c2", scaling: str = "weak") -> d
                                  "minibatch composition); the opt-in device-generated order is reported as *_device_order"}
 
 
+def dump_outputs(out_dir: str, algo, actor, critic, batch) -> None:
+    """What the caller of one headline step (``_preprocess_batch`` + ``_update_with_batch``) receives, as
+    ``out_dir/<name>.npy``: the per-minibatch loss table, the running return statistics, the actor's and the critic's
+    parameters, and the batch's per-transition ``v_s`` / ``returns`` / ``adv`` / ``logp_old``.  Rollouts longer than
+    ``DUMP_ROWS`` contribute the rows listed in ``row_index`` (a fixed seeded sample) instead of every row."""
+    import torch
+    rms = algo.ret_rms
+    out = {"loss_table": np.asarray(algo.last_loss_table, np.float64),
+           "ret_rms": np.concatenate([np.asarray(x, np.float64).reshape(-1) for x in (rms.mean, rms.var, rms.count)])}
+    for prefix, module in (("actor", actor), ("critic", critic)):
+        for name, p in module.named_parameters():
+            out[f"{prefix}.{name}"] = p.detach().float().cpu().numpy()
+    n = batch.obs.shape[0]
+    rows = None
+    if n > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+        out["row_index"] = rows.astype(np.float64)
+    for key in ("v_s", "returns", "adv", "logp_old"):
+        t = getattr(batch, key).detach()
+        if rows is not None:
+            t = t[torch.from_numpy(rows).to(t.device)]
+        out[key] = t.float().cpu().numpy()
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def positive_int(s: str) -> int:
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
+
+
 # ------------------------------------------------------------------------------------ GPU arm
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=positive_int, default=5, help="timed update() calls per timed arm")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
@@ -255,10 +297,14 @@ def main() -> None:
     ap.add_argument("--envs", type=int, default=0, help="override the config's env count (diagnostics)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip config4 / ingest / off-policy extras")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline arm computed as DIR/<name>.npy (rank 0)")
     ap.add_argument("--profile-one-step", action="store_true",
                     help="after the warm-up run ONE end-to-end update() between cudaProfilerStart/Stop and exit (for "
                          "`ncu --profile-from-start off ...`: the launch list of exactly the timed step)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -284,7 +330,7 @@ def main() -> None:
     assert world == args.gpus, f"--gpus {args.gpus} but WORLD_SIZE={world} (launch with torchrun)"
     _cabi.load_library()
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
     cfg = CONFIGS[args.config]
     E, T, BS = (args.envs or cfg["E"]), cfg["T"], cfg["bs"]
     N = E * T
@@ -363,6 +409,8 @@ def main() -> None:
         _cabi.reset_launch_count()
         ms_dev = timed(device_step, K)
         launches = _cabi.launch_count()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, algo, actor, critic, dev_batch)
         for _ in range(W):
             e2e_step()
         ms_e2e = timed(e2e_step, K)

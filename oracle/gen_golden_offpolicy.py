@@ -189,7 +189,9 @@ def gen_dqn():
                     out.update(named(algo.model_old, o + "qold_"))
             out[o + "tree_root"] = np.float64(buf.weight.reduce())
             out[o + "tree_leaves"] = np.asarray(buf.weight[np.arange(len(buf))]).copy()
+        params = {k: out.pop(k) for k in [k for k in out if k.startswith(f"u{cfg['updates'] - 1}_q")]}
         np.savez_compressed(os.path.join(OUT, f"dqn_ref{tag}.npz"), **out)
+        np.savez_compressed(os.path.join(OUT, f"dqn_ref{tag}_params.npz"), **params)     # apart: every file stays under 1 MB
         print(f"dqn_ref{tag}.npz", len(out), "arrays; losses", [float(out[f'u{u}_loss']) for u in range(cfg['updates'])])
 
 

@@ -68,7 +68,7 @@ def _worker(rank: int, world_size: int, port: int, variant: str, path: str, out_
 @pytest.mark.parametrize("variant", ["A", "B"])
 def test_two_rank_update_matches_reference(variant, path, tmp_path):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     import torch.multiprocessing as mp
     mp.spawn(_worker, args=(2, _free_port(), variant, path, str(tmp_path)), nprocs=2, join=True)
     a, b = torch.load(tmp_path / "flat0.pt"), torch.load(tmp_path / "flat1.pt")
@@ -82,7 +82,7 @@ def test_two_rank_shared_rollout_matches_reference(variant, tmp_path):
     Variant B's golden uses a minibatch size that does not divide the rollout (ragged last minibatch): a shared rollout
     refuses that split loudly (``ValueError`` from ``PPO._shared_slice``) instead of changing the minibatch composition."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     import torch.multiprocessing as mp
     if variant == "B":
         with pytest.raises(Exception, match="rollout_partition='shared' needs"):

@@ -1,90 +1,56 @@
-"""BASELINE configs[0] plumbing: the UNMODIFIED reference ``Collector`` + ``OnPolicyTrainer`` (imported from
-/root/reference through oracle/ref_shim.py) drive this package's ``Batch`` / ``VectorReplayBuffer`` /
-``DiscreteActorPolicy`` / ``OnPolicyAlgorithm`` on a 10-env CartPole-shaped environment for two epochs.
+"""BASELINE configs[0] plumbing: the UNMODIFIED reference ``Collector`` + ``OnPolicyTrainer`` drive this package's
+``Batch`` / ``VectorReplayBuffer`` / ``DiscreteActorPolicy`` / ``OnPolicyAlgorithm`` on a 10-env CartPole-shaped
+environment for two epochs.
 
-Runs on the build box only (the reference tree does not travel to the GPU box; there is no GPU here), so the numeric body
-of ``_update_with_batch`` is the numpy oracle (tests may use it) -- everything AROUND it is the product: the collector's
-``isinstance`` gates (collector.py:360,375-384) through ``tianshou_b200.compat``, ``buffer.add`` of the Collector's own
-Batch objects (:927-930), ``reset_buffer`` (trainer.py:1131), ``Algorithm.update`` with its training-step guard and lr
-scheduler (algorithm_base.py:586-631), the stats dataclass the trainer serialises (trainer.py:733-737,1122).
+tests/golden/integration_ref.npz (oracle/gen_golden_integration.py) is the call trace of that run: every ``buffer.add``
+the reference Collector made (its rows, buffer ids and what ``add`` returned), every ``buffer.reset`` of the trainer's
+``reset_buffer``, every ``algorithm.update`` the trainer made (arguments, numpy's generator state and learning rate at
+entry; mean loss and learning rate after it, parameters after the last one).  The test replays that sequence on fresh objects and checks that
+they return and compute what they did under the reference.  The numeric body of ``_update_with_batch`` is the numpy
+oracle (CPU test) -- everything AROUND it is the product: ``buffer.add`` of the Collector's rows (collector.py:927-930),
+``reset_buffer`` (trainer.py:1131), ``Algorithm.update`` with its training-step guard and lr scheduler
+(algorithm_base.py:586-631), the stats dataclass the trainer serialises (trainer.py:733-737,1122), and the
+``tianshou_b200.compat`` widening of the collector's ``isinstance`` gates (collector.py:360,375-384).
 """
 import dataclasses
+import types
 
 import numpy as np
 import pytest
 import torch
 
-from oracle.ref_shim import reference_available
+from ts_testutil import load_golden
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="needs the reference tree (build box only)")
-
-
-class FakeCartPole:
-    """CartPole-shaped stand-in (gymnasium is not installed): obs 4, 2 actions, reward 1 per step."""
-
-    metadata: dict = {}
-    spec = None
-
-    def __init__(self, seed: int = 0):
-        import gymnasium as gym        # the shim's stand-in spaces
-        self.action_space = gym.spaces.Discrete(2)
-        self.observation_space = gym.spaces.Box(-1.0, 1.0, (4,))
-        self.rng = np.random.default_rng(seed)
-        self.t = 0
-        self.unwrapped = self
-
-    def reset(self, seed=None, options=None):
-        self.t = 0
-        return self.rng.standard_normal(4).astype(np.float32), {}
-
-    def step(self, a):
-        self.t += 1
-        term = bool(self.rng.random() < 0.05)
-        return self.rng.standard_normal(4).astype(np.float32), 1.0, term, self.t >= 30 and not term, {}
-
-    def close(self):
-        pass
-
-    def seed(self, s=None):
-        return [s]
-
-    def render(self):
-        return None
+E = 10
+ADD_KEYS = ("obs", "act", "rew", "terminated", "truncated", "obs_next")
 
 
-def test_reference_collector_and_trainer_drive_b200_types():
+def params_of(actor, critic) -> dict:
+    """Every parameter of the shared-trunk actor / critic pair, by the numpy oracle's names."""
+    t1, t2 = [m for m in actor.preprocess.model.model if isinstance(m, torch.nn.Linear)]
+    a3, c3 = actor.last.model[0], critic.last.model[0]
+    return {"a_w1": t1.weight, "a_b1": t1.bias, "a_w2": t2.weight, "a_b2": t2.bias, "a_w3": a3.weight, "a_b3": a3.bias,
+            "c_w3": c3.weight, "c_b3": c3.bias}
+
+
+def build_oracle_ppo(action_space):
+    """This package's ``OnPolicyAlgorithm`` skeleton around a ``DiscreteActorPolicy``, with the numeric body of the update
+    from the numpy oracle (CPU stand-in for the kernels)."""
     from oracle import oracle_discrete as od
     from oracle import oracle_np as onp
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import gymnasium as gym
-    import tianshou.data.collector as refcol
-    from tianshou.env import DummyVectorEnv
-    from tianshou.trainer import OnPolicyTrainer, OnPolicyTrainerParams
-
-    import tianshou_b200.compat as compat
     from tianshou_b200.algorithm import A2CTrainingStats, AdamOptimizerFactory, DiscreteActorPolicy, OnPolicyAlgorithm
     from tianshou_b200.algorithm.optim import LRSchedulerFactoryLinear
-    from tianshou_b200.data import Batch, ReplayBufferManager, SequenceSummaryStats, VectorReplayBuffer
+    from tianshou_b200.data import Batch, SequenceSummaryStats, VectorReplayBuffer
     from tianshou_b200.utils.net.common import ActorCritic, Net
     from tianshou_b200.utils.net.discrete import DiscreteActor, DiscreteCritic
 
-    compat.install_into_reference()
-    compat.install_into_reference()                      # idempotent
-    assert ReplayBufferManager in refcol.ReplayBufferManager
-
-    torch.manual_seed(0)
-    np.random.seed(0)
-    E = 10
     net = Net(state_shape=(4,), hidden_sizes=(64, 64))
     actor = DiscreteActor(preprocess_net=net, action_shape=2, softmax_output=True)
     critic = DiscreteCritic(preprocess_net=net)
     policy = DiscreteActorPolicy(actor=actor, dist_fn=lambda p: torch.distributions.Categorical(probs=p),
-                                 action_space=gym.spaces.Discrete(2))
+                                 action_space=action_space)
 
     class OraclePPO(OnPolicyAlgorithm):
-        """This package's Algorithm skeleton with the numeric update body from the numpy oracle (CPU stand-in for the kernels)."""
-
         def __init__(self):
             super().__init__(policy=policy)
             self.critic = critic
@@ -94,12 +60,6 @@ def test_reference_collector_and_trainer_drive_b200_types():
             self.m = self.v = None
             self.step = 0
 
-        def _params(self):
-            t1, t2 = [m for m in actor.preprocess.model.model if isinstance(m, torch.nn.Linear)]
-            a3, c3 = actor.last.model[0], critic.last.model[0]
-            return {"a_w1": t1.weight, "a_b1": t1.bias, "a_w2": t2.weight, "a_b2": t2.bias, "a_w3": a3.weight, "a_b3": a3.bias,
-                    "c_w3": c3.weight, "c_b3": c3.bias}
-
         def _sample(self, buffer, sample_size):
             assert sample_size == 0 and isinstance(buffer, VectorReplayBuffer)
             idx = np.concatenate([np.arange(e * buffer._cap[e], e * buffer._cap[e] + buffer._sizes[e]) for e in range(E)])
@@ -108,7 +68,7 @@ def test_reference_collector_and_trainer_drive_b200_types():
         def _update_with_batch(self, batch, batch_size, repeat):
             assert self.policy.is_within_training_step and isinstance(batch, Batch)
             self.calls.append((len(batch), batch_size, repeat))
-            tp = self._params()
+            tp = params_of(actor, critic)
             p = {k: v.detach().numpy().copy() for k, v in tp.items()}
             if self.m is None:
                 self.m = {k: np.zeros_like(v) for k, v in p.items()}
@@ -139,21 +99,67 @@ def test_reference_collector_and_trainer_drive_b200_types():
             self._last_sizes = buffer._sizes.copy()
             return super().update(buffer, batch_size, repeat)
 
-    algo = OraclePPO()
+    return OraclePPO(), actor, critic
+
+
+def test_compat_widens_the_collector_gates():
+    import tianshou_b200.compat as compat
+    from tianshou_b200.algorithm.base import Algorithm
+    from tianshou_b200.data import ReplayBufferManager
+
+    class RefAlgorithm:                                  # the reference collector module's own names
+        pass
+
+    class RefReplayBufferManager:
+        pass
+
+    mod = types.SimpleNamespace(Algorithm=RefAlgorithm, ReplayBufferManager=RefReplayBufferManager)
+    compat.install_into_reference(mod)
+    compat.install_into_reference(mod)                   # idempotent
+    assert mod.Algorithm == (RefAlgorithm, Algorithm)
+    assert mod.ReplayBufferManager == (RefReplayBufferManager, ReplayBufferManager)
+
+
+def test_reference_collector_and_trainer_drive_b200_types():
+    from tianshou_b200.data import Batch, VectorReplayBuffer
+    from tianshou_b200.utils import policy_within_training_step
+
+    g = load_golden("integration_ref.npz")
+    algo, actor, critic = build_oracle_ppo(types.SimpleNamespace(n=2, shape=()))
+    with torch.no_grad():
+        for k, t in params_of(actor, critic).items():
+            t.copy_(torch.from_numpy(g["p0_" + k]))
     buf = VectorReplayBuffer(E * 40, E)
-    envs = DummyVectorEnv([lambda i=i: FakeCartPole(i) for i in range(E)])
-    collector = refcol.Collector(algo, envs, buf)                          # Algorithm -> .policy through the widened gate
-    assert collector.policy is policy and collector.buffer is buf
     w0 = actor.last.model[0].weight.detach().clone()
     with pytest.raises(RuntimeError):                                       # update outside a training step (algorithm_base.py:612-617)
         algo.update(buf, 64, 1)
-    params = OnPolicyTrainerParams(training_collector=collector, test_collector=None, max_epochs=2, epoch_num_steps=400,
-                                   collection_step_num_env_steps=200, batch_size=64, update_step_num_repetitions=2,
-                                   test_in_training=False, verbose=False, show_progress=False)
-    result = OnPolicyTrainer(algo, params).run()
+    n_add = n_reset = n_update = 0
+    for ev in g["events"]:
+        if ev == 0:
+            ret = buf.add(Batch(**{k: g["add_" + k][n_add] for k in ADD_KEYS}), buffer_ids=g["add_buffer_ids"][n_add])
+            for k, r in zip(("ptr", "ep_rew", "ep_len", "ep_idx"), ret, strict=True):
+                np.testing.assert_array_equal(np.asarray(r), g["add_ret_" + k][n_add], err_msg=f"add {n_add}: {k}")
+            n_add += 1
+        elif ev == 1:
+            buf.reset(keep_statistics=bool(g[f"reset{n_reset}_keep_statistics"]))
+            n_reset += 1
+        else:
+            o = f"update{n_update}_"
+            np.random.set_state(("MT19937", g[o + "np_key"], int(g[o + "np_pos"]), 0, 0.0))
+            assert algo.optim._optim.param_groups[0]["lr"] == float(g[o + "lr_before"])
+            with policy_within_training_step(algo.policy):
+                stats = algo.update(buf, int(g[o + "batch_size"]), int(g[o + "repeat"]))
+            assert algo.calls[-1][0] == int(g[o + "rows"])
+            assert stats.gradient_steps == int(g[o + "gradient_steps"])
+            np.testing.assert_allclose(stats.loss.mean, float(g[o + "loss_mean"]), rtol=1e-12, atol=1e-12)
+            np.testing.assert_allclose(algo.optim._optim.param_groups[0]["lr"], float(g[o + "lr_after"]), rtol=1e-12)
+            assert isinstance(dataclasses.asdict(stats), dict)
+            n_update += 1
+    assert n_add > 0 and n_reset > 0
+    for k, t in params_of(actor, critic).items():
+        np.testing.assert_allclose(t.detach().numpy(), g["final_p_" + k], rtol=1e-6, atol=1e-7, err_msg=k)
     assert len(algo.calls) == 4 and all(c[1:] == (64, 2) for c in algo.calls)          # 2 epochs x (400 / 200) update steps
     assert all(c[0] == 200 for c in algo.calls), algo.calls                             # the buffer was reset between collects
     assert not torch.equal(w0, actor.last.model[0].weight)                              # parameters moved
     assert algo.optim._optim.param_groups[0]["lr"] < 3e-4                               # lr scheduler stepped once per update()
-    assert isinstance(dataclasses.asdict(result), dict)
-    assert len(buf) == 0 or len(buf) <= E * 40
+    assert len(buf) <= E * 40

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 import torch
 
-from ts_testutil import load_golden, record_parity, set_buffer_state
+from ts_testutil import load_dqn_golden, load_golden, record_parity, set_buffer_state
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -162,7 +162,7 @@ def test_dqn_update_matches_reference(variant, mirror):
     replay: the frame stacks are gathered by the first convolution's im2col from the device copy of the frames."""
     from tianshou_b200.data import Batch, PrioritizedVectorReplayBuffer
     from tianshou_b200.utils import policy_within_training_step
-    g = load_golden(f"dqn_ref{variant}.npz")
+    g = load_dqn_golden(variant)
     algo, net, lr = _build_dqn(g)
     E, cap, steps = int(g["cfg_E"]), int(g["cfg_cap"]), int(g["cfg_steps"])
     buf = PrioritizedVectorReplayBuffer(E * cap, E, alpha=float(g["cfg_alpha"]), beta=float(g["cfg_beta"]), stack_num=4,

@@ -7,7 +7,7 @@ import pytest
 import torch
 
 from oracle import oracle_offpolicy as oo
-from ts_testutil import load_golden
+from ts_testutil import load_dqn_golden, load_golden
 
 
 def _load(params, g, prefix):
@@ -51,7 +51,7 @@ def test_sac_oracle_matches_reference_run():
 
 @pytest.mark.parametrize("variant", ["", "_b"])
 def test_dqn_oracle_matches_reference_run(variant):
-    g = load_golden(f"dqn_ref{variant}.npz")
+    g = load_dqn_golden(variant)
     H, W, A, E, cap = (int(g["cfg_" + k]) for k in ("H", "W", "A", "E", "cap"))
     lr = float(g["cfg_lr"])
     net = oo.nature_cnn(4, H, W, A)

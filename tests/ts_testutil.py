@@ -14,6 +14,12 @@ def load_golden(name: str):
     return np.load(os.path.join(GOLDEN, name), allow_pickle=False)
 
 
+def load_dqn_golden(variant: str) -> dict:
+    """``dqn_ref{variant}.npz`` together with ``dqn_ref{variant}_params.npz`` (the network parameters after the last
+    update, stored in a file of their own so that no fixture file exceeds 1 MB)."""
+    return {**load_golden(f"dqn_ref{variant}.npz"), **load_golden(f"dqn_ref{variant}_params.npz")}
+
+
 PARAM_ORDER = ["a_w1", "a_b1", "a_w2", "a_b2", "a_w3", "a_b3", "a_logstd",
                "c_w1", "c_b1", "c_w2", "c_b2", "c_w3", "c_b3"]
 
