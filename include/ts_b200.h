@@ -475,8 +475,20 @@ int ts_dqn_loss(const float* q, const int64_t* act, const float* returns, const 
 /* DQN._target_q (dqn.py:365-380): double -> q_target[b][argmax_a q_online[b][a]], else max_a q_target[b][a] */
 int ts_dqn_target(const float* q_online, const float* q_target, int64_t B, int32_t A, int32_t is_double, float* out,
                   ts_stream_t stream);
-/* min(q1, q2) - alpha * logp   (td3.py:94-102, sac.py:298-302) */
+/* min(q1, q2) - alpha * logp   (td3.py:94-102, sac.py:298-302).  logp == NULL means no entropy term: out = min(q1, q2),
+ * TD3's target value (td3.py:94-102); alpha is then ignored. */
 int ts_sac_target(const float* q1, const float* q2, const float* logp, float alpha, int64_t B, float* out, ts_stream_t stream);
+/* ContinuousActorDeterministic.forward (utils/net/continuous.py:70-85) on the last Linear's output z[B][A] (row stride ld):
+ * act = max_action * tanh(z).  With noise != NULL (a [B][A] standard-normal draw) TD3's target-policy smoothing
+ * (td3.py:190-202): n = noise * policy_noise, clamped to [-noise_clip, noise_clip] if noise_clip > 0, act += n; the smoothed
+ * action is not clamped to the action bounds, as in the reference.  act is dense [B][A]. */
+int ts_det_actor_head(const float* z, int64_t ld, int64_t B, int32_t A, float max_action, const float* noise, float policy_noise,
+                      float noise_clip, float* act, ts_stream_t stream);
+/* backward of the head: dz = dact * max_action * (1 - tanh(z)^2), dz in the layout of z (utils/net/continuous.py:84) */
+int ts_det_actor_head_bwd(const float* z, int64_t ld, const float* dact, int64_t B, int32_t A, float max_action, float* dz,
+                          ts_stream_t stream);
+/* DDPG / TD3 actor loss -critic(obs, actor(obs)).mean() (ddpg.py:406, td3.py:216): loss_rows = -q, dq = -1 / B */
+int ts_det_actor_q_grad(const float* q, int64_t B, float* dq, float* loss_rows, ts_stream_t stream);
 /* rows of alpha*logp - min(q1,q2) and d(-min)/dq / B with torch.minimum's tie rule (sac.py:315-321) */
 int ts_sac_actor_q_grad(const float* q1, const float* q2, const float* logp, float alpha, int64_t B, float* dq1, float* dq2,
                         float* loss_rows, ts_stream_t stream);

@@ -122,6 +122,9 @@ SIGNATURES: dict[str, list[Any]] = {
     "ts_dqn_target": [_P, _P, _I64, _I32, _I32, _P, _P],
     "ts_sac_target": [_P, _P, _P, C.c_float, _I64, _P, _P],
     "ts_sac_actor_q_grad": [_P, _P, _P, C.c_float, _I64, _P, _P, _P, _P],
+    "ts_det_actor_head": [_P, _I64, _I64, _I32, C.c_float, _P, C.c_float, C.c_float, _P, _P],
+    "ts_det_actor_head_bwd": [_P, _I64, _P, _I64, _I32, C.c_float, _P, _P],
+    "ts_det_actor_q_grad": [_P, _I64, _P, _P, _P],
     "ts_mean": [_P, _I64, _P, _P],
     "ts_adam_step": [_P, _P, _P, _P, _I64, _I64, _D, _D, _D, _D, _D, _D, _P, _P],
     "ts_adam_step_dev": [_P, _P, _P, _P, _I64, _P, _D, _D, _D, _D, _D, _D, _P, _P],

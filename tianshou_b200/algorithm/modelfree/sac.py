@@ -11,11 +11,11 @@ Per ``update(buffer, sample_size)``:
          forward -> ``ts_sac_target`` -> ``ts_nstep_return``; per critic forward / loss / backward (``ts_net_gemm``) + Adam;
          actor forward, critics' input-gradient GEMMs, tanh-Gaussian head backward, actor backward + Adam; Polyak axpy.
 Every Linear layer's forward / input gradient / weight gradient is one tcgen05 GEMM launch (csrc/net_gemm.cu).
+The row gathers, critic step, Polyak update and CUDA-graph mode are shared with DDPG / TD3 (ddpg.py, td3.py).
 """
 from __future__ import annotations
 
 from abc import ABC, abstractmethod
-from copy import deepcopy
 from dataclasses import dataclass
 from typing import Any, Union
 
@@ -24,12 +24,14 @@ import torch
 from torch import nn
 from torch.distributions import Independent, Normal
 
-from ..._cabi import call, ptr, stream_ptr, to_device
+from ..._cabi import call, ptr, stream_ptr
 from ...data import Batch, ReplayBuffer
-from ..base import OffPolicyAlgorithm, Policy, TrainingStats
+from ..base import Policy, TrainingStats
 from ..flat_params import UnsupportedModelError
-from ..netgraph import ACT_NONE, FlatGroup, FusedStack, _Layer, compile_sequential, module_layers, polyak_update
+from ..netgraph import ACT_NONE, _Layer
 from ..optim import OptimizerFactory
+from .ddpg import _linear_relu_chain, describe_q_critic  # noqa: F401  (describe_q_critic: re-exported)
+from .td3 import ActorDualCriticsOffPolicyAlgorithm
 
 SIGMA_MIN, SIGMA_MAX = -20.0, 2.0          # utils/net/continuous.py:17-18
 _F32_EPS = float(np.finfo(np.float32).eps)
@@ -136,29 +138,6 @@ class AutoAlpha(nn.Module, Alpha):
 
 
 # ------------------------------------------------------------------------------------------------ module -> kernel views
-def _linear_relu_chain(mod: Any, in_dim: int, what: str) -> list[_Layer]:
-    try:
-        return compile_sequential(module_layers(mod), (in_dim,))
-    except UnsupportedModelError as e:
-        raise UnsupportedModelError(f"{what}: {e}") from e
-
-
-def describe_q_critic(critic: Any, obs_dim: int, act_dim: int) -> tuple[list[_Layer], list[nn.Parameter]]:
-    """ContinuousCritic(preprocess_net=Net(concat=True), ...) -> Linear/ReLU chain on concat(obs, act) ending in 1 output."""
-    if getattr(critic, "apply_preprocess_net_to_obs_only", False):
-        raise UnsupportedModelError("critic: apply_preprocess_net_to_obs_only unsupported")
-    layers = _linear_relu_chain(critic.preprocess, obs_dim + act_dim, "critic.preprocess")
-    if getattr(critic.preprocess, "softmax", False):
-        raise UnsupportedModelError("critic: softmax trunk output unsupported")
-    layers += _linear_relu_chain(critic.last, layers[-1].out_dim, "critic.last")
-    if layers[-1].out_dim != 1 or layers[-1].act != ACT_NONE:
-        raise UnsupportedModelError("critic must end in a single linear Q output")
-    params: list[nn.Parameter] = []
-    for L in layers:
-        params += [L.weight, L.bias]
-    return layers, params
-
-
 def describe_gaussian_actor(actor: Any, obs_dim: int) -> tuple[list[_Layer], list[nn.Parameter], int]:
     """ContinuousActorProbabilistic(conditioned_sigma=True, unbounded=True): trunk + ONE virtual head layer whose rows are
     (mu.weight ; sigma.weight) -- adjacent in the flat buffer, so the head is a single [2A, H] GEMM."""
@@ -180,81 +159,26 @@ def describe_gaussian_actor(actor: Any, obs_dim: int) -> tuple[list[_Layer], lis
     return [*trunk, head], params, A
 
 
-class SAC(OffPolicyAlgorithm):
+class SAC(ActorDualCriticsOffPolicyAlgorithm):
     """Soft Actor-Critic (arXiv:1801.01290 / 1812.05905), reference API (sac.py:218-336)."""
+
+    _n_noise = 2        # the two rsample draws: target action, then the actor step's action
+    _n_losses = 3
 
     def __init__(self, *, policy: SACPolicy, policy_optim: OptimizerFactory, critic: nn.Module, critic_optim: OptimizerFactory,
                  critic2: nn.Module | None = None, critic2_optim: OptimizerFactory | None = None, tau: float = 0.005,
                  gamma: float = 0.99, alpha: float | Alpha = 0.2, n_step_return_horizon: int = 1,
                  deterministic_eval: bool = True, cuda_graph: bool = False) -> None:
-        assert 0.0 <= tau <= 1.0, f"tau should be in [0, 1] but got: {tau}"
-        assert 0.0 <= gamma <= 1.0, f"gamma should be in [0, 1] but got: {gamma}"
-        super().__init__(policy=policy)
-        if _space_name(policy.action_space) != "continuous":
-            raise ValueError(f"SACPolicy only supports Box action spaces, but got {policy.action_space=}.")
-        self.tau = tau
-        self.gamma = gamma
-        self.n_step_return_horizon = n_step_return_horizon
+        super().__init__(policy=policy, policy_optim=policy_optim, critic=critic, critic_optim=critic_optim, critic2=critic2,
+                         critic2_optim=critic2_optim, tau=tau, gamma=gamma, n_step_return_horizon=n_step_return_horizon,
+                         cuda_graph=cuda_graph)
         self.deterministic_eval = deterministic_eval
         self.alpha = Alpha.from_float_or_instance(alpha)
-        self.critic = critic
-        self.critic2 = critic2 or deepcopy(critic)
-        self.critic_old = deepcopy(self.critic).eval()
-        self.critic2_old = deepcopy(self.critic2).eval()
-        dev = next(policy.actor.parameters()).device
-        if dev.type != "cuda":
-            raise UnsupportedModelError(f"networks live on {dev}; tianshou_b200 has no CPU path -- move them to a CUDA device")
-        self._dev = dev
-        first = module_layers(policy.actor.preprocess)[0]
-        self.obs_dim = int(first.in_features)
-        a_layers, a_params, self.act_dim = describe_gaussian_actor(policy.actor, self.obs_dim)
-        self._g_actor = FlatGroup(a_params, dev)
-        self._actor = FusedStack(a_layers, self._g_actor, "actor")
-        self._g_c, self._c, self._g_ct = [], [], []
-        for src, tgt in ((self.critic, self.critic_old), (self.critic2, self.critic2_old)):
-            layers, params = describe_q_critic(src, self.obs_dim, self.act_dim)
-            _, tparams = describe_q_critic(tgt, self.obs_dim, self.act_dim)
-            g = FlatGroup(params, dev)
-            self._g_c.append(g)
-            self._c.append(FusedStack(layers, g, "critic"))
-            self._g_ct.append(FlatGroup(tparams, dev))
-        self.policy_optim = self._create_optimizer(policy, policy_optim)
-        self.critic_optim = self._create_optimizer(self.critic, critic_optim)
-        self.critic2_optim = self._create_optimizer(self.critic2, critic2_optim or critic_optim)
-        for o, g in ((self.policy_optim, self._g_actor), (self.critic_optim, self._g_c[0]), (self.critic2_optim, self._g_c[1])):
-            if set(map(id, o._optim.param_groups[0]["params"])) != set(map(id, g.params)):
-                raise UnsupportedModelError("optimizer parameters differ from the fused network's parameters")
-            o._flat = g
-        self._scratch: dict[str, torch.Tensor] = {}
-        # opt-in: the device work of one update() (~85 launches) captured once into a CUDA graph and replayed -- the eager call
-        # sequence is Python-launch bound.  Needs a buffer with a device mirror, uniform replay and a fixed alpha.
-        self.cuda_graph = bool(cuda_graph)
-        self._graph: dict[str, Any] = {}
-        self._adam = FlatGroup.adam_step          # the graphed body switches to the device-step variant
-        # rsample noise source: torch's generator on the networks' device (what the reference draws when it runs there)
-        self._noise_fn = lambda shape: torch.normal(torch.zeros(shape, device=dev), torch.ones(shape, device=dev))
+
+    def _describe_actor(self, actor: nn.Module) -> tuple[list[_Layer], list[nn.Parameter], int]:
+        return describe_gaussian_actor(actor, self.obs_dim)
 
     # ------------------------------------------------------------------ helpers
-    def _buf(self, name: str, shape: tuple[int, ...] | int, dtype: torch.dtype = torch.float32) -> torch.Tensor:
-        shape = (shape,) if isinstance(shape, int) else tuple(shape)
-        t = self._scratch.get(name)
-        if t is None or t.shape != shape or t.dtype != dtype:
-            t = self._scratch[name] = torch.empty(shape, dtype=dtype, device=self._dev)
-        return t
-
-    def _rows(self, buffer: ReplayBuffer, key: str, indices: np.ndarray | torch.Tensor) -> torch.Tensor:
-        """buffer[key][indices] as a dense fp32 [I, width] device tensor: gathered from the device mirror when the
-        buffer keeps one (no host traffic), else a host gather of the sampled rows + one upload."""
-        cols = self._cols_override if self._cols_override is not None else (
-            buffer.device_columns() if hasattr(buffer, "device_columns") else None)
-        if cols is not None and key in cols:
-            from ... import ops
-            idx = indices if isinstance(indices, torch.Tensor) else to_device(np.asarray(indices, dtype=np.int64), self._dev)
-            src = cols[key]
-            return ops.gather_rows(src.reshape(src.shape[0], -1), idx).to(torch.float32)
-        arr = np.asarray(buffer._meta[key])[np.asarray(indices)]
-        return to_device(np.ascontiguousarray(arr.reshape(len(arr), -1)), self._dev, dtype=torch.float32)
-
     def _actor_forward(self, obs: torch.Tensor, tag: str) -> tuple[list[torch.Tensor], torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
         """policy(batch) on the device: returns (activations, act, log_prob, sigma, noise)."""
         B, A = obs.shape[0], self.act_dim
@@ -268,72 +192,24 @@ class SAC(OffPolicyAlgorithm):
              ptr(sigma), stream_ptr(self._dev))
         return acts, act, logp, sigma, noise
 
-    def _q_forward(self, k: int, obs: torch.Tensor, act: torch.Tensor, tag: str, target: bool = False) -> tuple[list[torch.Tensor], torch.Tensor]:
-        B = obs.shape[0]
-        x = self._buf(f"{tag}_x{k}", (B, self.obs_dim + self.act_dim))
-        call("ts_concat2", ptr(obs), self.obs_dim, ptr(act), self.act_dim, B, ptr(x), stream_ptr(self._dev))
-        if target:
-            self._g_ct[k].ensure_adopted()
-        acts = self._c[k].forward(x, B, tag, params=self._g_ct[k].flat if target else None)
-        return acts, acts[-1].view(B)
-
     # ------------------------------------------------------------------ target
     def _target_q(self, buffer: ReplayBuffer, indices: np.ndarray) -> torch.Tensor:
         """min(Q1', Q2')(s', a') - alpha * log pi(a'|s') with a' ~ pi(.|s')   (ddpg.py:327-339, td3.py:94-102, sac.py:298-302)"""
-        if buffer._save_obs_next:
-            obs_next = self._rows(buffer, "obs_next", indices)
-        else:
-            obs_next = self._rows(buffer, "obs", buffer.next(indices))
+        obs_next = self._obs_next(buffer, indices)
         B = obs_next.shape[0]
-        _, act, logp, _, _ = self._actor_forward(obs_next.contiguous(), "tq")
+        _, act, logp, _, _ = self._actor_forward(obs_next, "tq")
         _, q1 = self._q_forward(0, obs_next, act, "tq", target=True)
         _, q2 = self._q_forward(1, obs_next, act, "tq", target=True)
         out = self._buf("tq_out", (B, 1))
         call("ts_sac_target", ptr(q1), ptr(q2), ptr(logp), float(self.alpha.value), B, ptr(out), stream_ptr(self._dev))
         return out
 
-    def _preprocess_batch(self, batch: Batch, buffer: ReplayBuffer, indices: np.ndarray) -> Batch:
-        return self.compute_nstep_return(batch=batch, buffer=buffer, indices=indices, target_q_fn=self._target_q,
-                                         gamma=self.gamma, n_step=self.n_step_return_horizon)
-
-    def _sample(self, buffer: ReplayBuffer, sample_size: int | None) -> tuple[Batch, Any]:
-        """Indices from the buffer's host RNG streams (identical to the reference's draws); rows stay on the device."""
-        indices = buffer.sample_indices(sample_size)
-        batch = Batch()
-        batch.__dict__["obs"] = self._rows(buffer, "obs", indices).contiguous()
-        batch.__dict__["act"] = self._rows(buffer, "act", indices).contiguous()
-        if hasattr(buffer, "get_weight"):          # PrioritizedReplayBuffer.__getitem__ adds the IS weight (prio.py:104-106)
-            w = buffer.get_weight(indices)
-            batch.__dict__["weight"] = to_device(np.asarray(w / np.max(w) if buffer._weight_norm else w, dtype=np.float32), self._dev)
-        batch.__dict__["info"] = Batch()
-        return batch, indices
-
     # ------------------------------------------------------------------ update
-    def _critic_step(self, k: int, obs: torch.Tensor, act: torch.Tensor, returns: torch.Tensor, weight: torch.Tensor | None,
-                     optim: Any, out_loss: torch.Tensor) -> torch.Tensor:
-        """``_minimize_critic_squared_loss`` (ddpg.py:267-285): forward, weighted MSE, backward, Adam."""
-        B = obs.shape[0]
+    def _update_with_batch(self, batch: Batch) -> SACTrainingStats | None:
         st = stream_ptr(self._dev)
-        acts, q = self._q_forward(k, obs, act, "cu")
-        td = self._buf(f"td{k}", B)
-        dq = self._buf("dq", (B, 1))
-        rows = self._buf("loss_rows", B)
-        call("ts_critic_mse", ptr(q), ptr(returns), ptr(weight), B, ptr(td), ptr(dq), ptr(rows), st)
-        call("ts_mean", ptr(rows), B, ptr(out_loss), st)
-        self._c[k].backward(acts, dq, B, "cu")
-        self._adam(self._g_c[k], optim._optim, optim._max_grad_norm)
-        return td
-
-    def _update_with_batch(self, batch: Batch) -> SACTrainingStats:
-        dev, st = self._dev, stream_ptr(self._dev)
         obs, act = batch.obs, batch.act
         B, A = obs.shape[0], self.act_dim
-        returns = batch.returns.reshape(-1).to(dev, torch.float32).contiguous()
-        weight = getattr(batch, "weight", None)
-        if weight is not None and not isinstance(weight, torch.Tensor):
-            weight = to_device(np.asarray(weight, dtype=np.float32), dev)
-        if weight is not None:
-            weight = weight.reshape(-1).to(dev, torch.float32).contiguous()
+        returns, weight = self._returns_and_weight(batch)
         losses = self._buf("losses", 3)
         td1 = self._critic_step(0, obs, act, returns, weight, self.critic_optim, losses[0:1])
         td2 = self._critic_step(1, obs, act, returns, weight, self.critic2_optim, losses[1:2])
@@ -358,107 +234,15 @@ class SAC(OffPolicyAlgorithm):
         self._adam(self._g_actor, self.policy_optim._optim, self.policy_optim._max_grad_norm)
 
         alpha_loss = None if self._in_graph_body else self.alpha.update(-logp.detach().unsqueeze(-1))
-        for k in range(2):                      # _update_lagged_network_weights
-            polyak_update(self._g_ct[k], self._g_c[k], self.tau)
+        self._update_lagged_network_weights()
         if self._in_graph_body:
             return None                         # the losses stay on the device; update() reads them after the replay
-        l = losses.cpu().numpy()                # the only host sync of the update
-        return SACTrainingStats(actor_loss=float(l[2]), critic1_loss=float(l[0]), critic2_loss=float(l[1]),
+        return self._stats_from_losses(losses.cpu().numpy(), alpha_loss)      # the only host sync of the update
+
+    def _stats_from_losses(self, losses: np.ndarray, alpha_loss: float | None = None) -> SACTrainingStats:
+        return SACTrainingStats(actor_loss=float(losses[2]), critic1_loss=float(losses[0]), critic2_loss=float(losses[1]),
                                 alpha=float(self.alpha.value), alpha_loss=alpha_loss)
 
     # ------------------------------------------------------------------ CUDA-graph mode
-    _in_graph_body = False
-    _cols_override: Any = None          # the mirror's columns while the graphed body runs (no cross-stream wait inside a capture)
-
     def _graph_usable(self, buffer: ReplayBuffer) -> bool:
-        cols = buffer.device_columns() if hasattr(buffer, "device_columns") else None
-        # (a learning-rate schedule would change a constant baked into the captured launches every update: eager then)
-        return (self.cuda_graph and isinstance(self.alpha, FixedAlpha) and not hasattr(buffer, "update_weight") and cols is not None
-                and not self.lr_schedulers
-                and buffer._save_obs_next and all(k in cols for k in ("obs", "act", "rew", "terminated", "done", "obs_next")))
-
-    def _device_body(self, buffer: ReplayBuffer, g: dict[str, Any]) -> None:
-        """Everything of one update() after the index / noise draws, with no host synchronisation: n-step chain, target,
-        both critic steps, the actor step, Polyak.  Runs eagerly once, then inside the capture, then as graph replays."""
-        from ... import ops
-        idx, meta, cols = g["idx"], g["meta"], g["cols"]
-        noise_iter = iter((g["noise"][0], g["noise"][1]))
-        saved_fn, self._noise_fn = self._noise_fn, lambda shape: next(noise_iter)
-        saved_adam, self._adam = self._adam, FlatGroup.adam_step_device
-        self._in_graph_body, self._cols_override = True, cols
-        try:
-            B = idx.numel()
-            n = self.n_step_return_horizon
-            stacked = ops.stack_next_indices(meta, idx, n)
-            last = stacked[-1].contiguous()
-            tq = self._target_q(buffer, last).reshape(B, -1).clone()
-            ops.value_mask_rows(tq, cols["terminated"].view(torch.uint8), last)
-            rew = cols["rew"] if cols["rew"].dtype == torch.float64 else cols["rew"].to(torch.float64)
-            returns = ops.nstep_return(rew, ops.buffer_end_flags(meta), tq, stacked, self.gamma, n, out_dtype=torch.float64)
-            batch = Batch()
-            batch.__dict__["obs"] = self._rows(buffer, "obs", idx).contiguous()
-            batch.__dict__["act"] = self._rows(buffer, "act", idx).contiguous()
-            batch.__dict__["returns"] = returns.to(torch.float32)
-            self._update_with_batch(batch)
-            g["h_losses"].copy_(self._buf("losses", 3), non_blocking=True)
-        finally:
-            self._noise_fn, self._adam, self._in_graph_body, self._cols_override = saved_fn, saved_adam, False, None
-
-    def update(self, buffer: ReplayBuffer, sample_size: int | None) -> TrainingStats:
-        """``OffPolicyAlgorithm.update`` (algorithm_base.py:868-903); with ``cuda_graph=True`` the device work is one graph replay."""
-        if buffer is None or not self.policy.is_within_training_step or not self._graph_usable(buffer):
-            return super().update(buffer, sample_size)
-        import time
-
-        from ...ops import DeviceBufferMeta
-        from ...utils.torch_utils import torch_train_mode
-        start = time.time()
-        dev = self._dev
-        indices = np.asarray(buffer.sample_indices(sample_size), dtype=np.int64)
-        B, A = len(indices), self.act_dim
-        cols = buffer.device_columns()                       # also orders this stream after the mirror's pending copies
-        E = int(buffer.buffer_num)
-        g = self._graph
-        key = (B, E, tuple(int(cols[k].data_ptr()) for k in sorted(cols)), float(self.policy_optim._optim.param_groups[0]["lr"]),
-               float(self.critic_optim._optim.param_groups[0]["lr"]), float(self.critic2_optim._optim.param_groups[0]["lr"]))
-        if g.get("key") != key:                              # (re)build the persistent inputs; the next call captures
-            g.clear()
-            g.update(key=key, calls=0, graph=None, cols=dict(cols),
-                     h_idx=torch.empty(B, dtype=torch.int64, pin_memory=True), idx=torch.empty(B, dtype=torch.int64, device=dev),
-                     h_meta=torch.empty((3, E), dtype=torch.int64, pin_memory=True), d_meta=torch.empty((3, E), dtype=torch.int64, device=dev),
-                     noise=torch.empty((2, B, A), dtype=torch.float32, device=dev), h_losses=torch.empty(3, dtype=torch.float32, pin_memory=True))
-            off = torch.from_numpy(np.asarray(buffer._extend_offset, dtype=np.int64)).to(dev)
-            g["meta"] = DeviceBufferMeta(off, cols["done"].view(torch.uint8), g["d_meta"][0], g["d_meta"][1], g["d_meta"][2])
-        g["h_idx"].numpy()[...] = indices
-        hm = g["h_meta"].numpy()
-        hm[0], hm[1], hm[2] = buffer.last_index, buffer._sizes, buffer._ins
-        g["idx"].copy_(g["h_idx"], non_blocking=True)
-        g["d_meta"].copy_(g["h_meta"], non_blocking=True)
-        g["noise"][0].copy_(self._noise_fn((B, A)).to(dev, torch.float32))      # the two rsample draws, in the reference's order
-        g["noise"][1].copy_(self._noise_fn((B, A)).to(dev, torch.float32))
-        with torch_train_mode(self):
-            if g["graph"] is not None:
-                g["graph"].replay()
-            elif g["calls"] == 0:                            # first update with these shapes: eager (allocates every scratch buffer)
-                self._device_body(buffer, g)
-            else:                                            # second: capture, then replay it as this update
-                graph = torch.cuda.CUDAGraph()
-                torch.cuda.synchronize(dev)
-                with torch.cuda.graph(graph):
-                    self._device_body(buffer, g)
-                g["graph"] = graph
-                graph.replay()
-        g["calls"] += 1
-        torch.cuda.current_stream(dev).synchronize()         # the one host sync: the three loss scalars
-        l = g["h_losses"].numpy()
-        for sched in self.lr_schedulers:
-            sched.step()
-        stat = SACTrainingStats(actor_loss=float(l[2]), critic1_loss=float(l[0]), critic2_loss=float(l[1]), alpha=float(self.alpha.value),
-                                alpha_loss=None)
-        stat.train_time = time.time() - start
-        return stat
-
-
-def _space_name(space: Any) -> str:
-    from ..base import _space_kind
-    return _space_kind(space)
+        return isinstance(self.alpha, FixedAlpha) and super()._graph_usable(buffer)

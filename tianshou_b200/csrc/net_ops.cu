@@ -5,7 +5,8 @@
 //
 // Reference code replaced: ReplayBuffer.get frame stacking (data/buffer/buffer_base.py:557-603), DQNet conv stack
 // (env/atari/atari_network.py:77-84), SACPolicy.forward tanh-squashed Gaussian (modelfree/sac.py:108-131),
-// SAC actor / critic losses (sac.py:304-322, ddpg.py:279-285), DQN loss (dqn.py:384-401), torch.optim.Adam
+// SAC actor / critic losses (sac.py:304-322, ddpg.py:279-285), the deterministic actor head of DDPG / TD3 with TD3's
+// target-policy smoothing (utils/net/continuous.py:70-85, td3.py:190-202) and their actor loss (ddpg.py:406, td3.py:216), DQN loss (dqn.py:384-401), torch.optim.Adam
 // single-tensor step (optim.py:89-110), polyak_parameter_update (utils/lagged_network.py:8-18).
 #include <math.h>
 
@@ -232,12 +233,48 @@ __global__ void dqn_target_kernel(const float* __restrict__ q_online, const floa
     for (int a = 1; a < A; ++a) { const float v = src[b * A + a]; if (v > bv) { bv = v; best = a; } }
     out[b] = q_target[b * A + best];
 }
-// SAC target: min(q1, q2) - alpha * logp   (td3.py:94-102, sac.py:298-302)
+// SAC target: min(q1, q2) - alpha * logp   (td3.py:94-102, sac.py:298-302); logp == nullptr: min(q1, q2) alone (TD3)
 __global__ void sac_target_kernel(const float* __restrict__ q1, const float* __restrict__ q2, const float* __restrict__ logp, float alpha,
                                   int64_t B, float* __restrict__ out) {
     const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
-    out[b] = fminf(q1[b], q2[b]) - alpha * logp[b];
+    out[b] = logp ? fminf(q1[b], q2[b]) - alpha * logp[b] : fminf(q1[b], q2[b]);
+}
+
+// ---- deterministic actor head (ContinuousActorDeterministic.forward, utils/net/continuous.py:70-85) ----------------------
+// act = max_action * tanh(z); with `noise` (TD3 target-policy smoothing, td3.py:190-202): n = noise * policy_noise, clamped to
+// [-noise_clip, noise_clip] when noise_clip > 0, act += n.  The smoothed action is not clamped to the action bounds (nor is it
+// in the reference).  One thread per element: B * A elements, row stride ld of z.
+__global__ void det_actor_head_kernel(const float* __restrict__ z, int64_t ld, int64_t B, int A, float max_action,
+                                      const float* __restrict__ noise, float policy_noise, float noise_clip, float* __restrict__ act) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= B * A) return;
+    const int64_t b = t / A;
+    const int a = (int)(t - b * A);
+    float y = max_action * tanhf(z[b * ld + a]);
+    if (noise) {
+        float n = noise[t] * policy_noise;
+        if (noise_clip > 0.0f) n = fminf(fmaxf(n, -noise_clip), noise_clip);
+        y += n;
+    }
+    act[t] = y;
+}
+// dz = dact * max_action * (1 - tanh(z)^2): the gradient at the last Linear's output (layout of z)
+__global__ void det_actor_head_bwd_kernel(const float* __restrict__ z, int64_t ld, const float* __restrict__ dact, int64_t B, int A,
+                                          float max_action, float* __restrict__ dz) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= B * A) return;
+    const int64_t b = t / A;
+    const int a = (int)(t - b * A);
+    const float th = tanhf(z[b * ld + a]);
+    dz[b * ld + a] = dact[t] * max_action * (1.0f - th * th);
+}
+// DDPG / TD3 actor loss -Q(s, actor(s)).mean() (ddpg.py:406, td3.py:216): loss rows -q, dq = -1 / B
+__global__ void det_actor_q_grad_kernel(const float* __restrict__ q, int64_t B, float* __restrict__ dq, float* __restrict__ loss_rows) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    dq[b] = -1.0f / (float)B;
+    loss_rows[b] = -q[b];
 }
 // d(-min(q1, q2))/d(q1, q2) / B with torch.minimum's tie rule (equal -> half each); also the actor-loss rows
 __global__ void sac_actor_q_grad_kernel(const float* __restrict__ q1, const float* __restrict__ q2, const float* __restrict__ logp, float alpha,
@@ -412,8 +449,22 @@ extern "C" int ts_dqn_target(const float* q_online, const float* q_target, int64
     TS_LAUNCH_1D(dqn_target_kernel, B, q_online, q_target, B, A, is_double, out);
 }
 extern "C" int ts_sac_target(const float* q1, const float* q2, const float* logp, float alpha, int64_t B, float* out, ts_stream_t stream) {
-    TS_REQUIRE(q1 && q2 && logp && out, "ts_sac_target: null pointer");
+    TS_REQUIRE(q1 && q2 && out, "ts_sac_target: null pointer");
     TS_LAUNCH_1D(sac_target_kernel, B, q1, q2, logp, alpha, B, out);
+}
+extern "C" int ts_det_actor_head(const float* z, int64_t ld, int64_t B, int32_t A, float max_action, const float* noise,
+                                 float policy_noise, float noise_clip, float* act, ts_stream_t stream) {
+    TS_REQUIRE(z && act && A >= 1 && ld >= (int64_t)A, "ts_det_actor_head: bad argument");
+    TS_LAUNCH_1D(det_actor_head_kernel, B * A, z, ld, B, A, max_action, noise, policy_noise, noise_clip, act);
+}
+extern "C" int ts_det_actor_head_bwd(const float* z, int64_t ld, const float* dact, int64_t B, int32_t A, float max_action, float* dz,
+                                     ts_stream_t stream) {
+    TS_REQUIRE(z && dact && dz && A >= 1 && ld >= (int64_t)A, "ts_det_actor_head_bwd: bad argument");
+    TS_LAUNCH_1D(det_actor_head_bwd_kernel, B * A, z, ld, dact, B, A, max_action, dz);
+}
+extern "C" int ts_det_actor_q_grad(const float* q, int64_t B, float* dq, float* loss_rows, ts_stream_t stream) {
+    TS_REQUIRE(q && dq && loss_rows, "ts_det_actor_q_grad: null pointer");
+    TS_LAUNCH_1D(det_actor_q_grad_kernel, B, q, B, dq, loss_rows);
 }
 extern "C" int ts_sac_actor_q_grad(const float* q1, const float* q2, const float* logp, float alpha, int64_t B, float* dq1, float* dq2,
                                    float* loss_rows, ts_stream_t stream) {

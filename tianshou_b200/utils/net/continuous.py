@@ -1,4 +1,4 @@
-"""Gaussian actor / state-value critic heads (API of tianshou/utils/net/continuous.py:96-238)."""
+"""Deterministic and Gaussian actors, critic heads (API of tianshou/utils/net/continuous.py:32-238)."""
 from __future__ import annotations
 
 import warnings
@@ -41,6 +41,24 @@ class ContinuousCritic(ModuleWithVectorOutput):
         if not self.apply_preprocess_net_to_obs_only:
             obs, _ = self.preprocess(obs)
         return self.last(obs)
+
+
+class ContinuousActorDeterministic(ModuleWithVectorOutput):
+    """Actions directly (DDPG / TD3): preprocess net -> ``last`` MLP -> ``max_action * tanh`` (continuous.py:32-85)."""
+
+    def __init__(self, *, preprocess_net: ModuleWithVectorOutput, action_shape: Any, hidden_sizes: Sequence[int] = (),
+                 max_action: float = 1.0) -> None:
+        super().__init__(int(np.prod(action_shape)))
+        self.preprocess = preprocess_net
+        self.last = MLP(input_dim=preprocess_net.get_output_dim(), output_dim=self.output_dim, hidden_sizes=hidden_sizes)
+        self.max_action = max_action
+
+    def get_preprocess_net(self) -> ModuleWithVectorOutput:
+        return self.preprocess
+
+    def forward(self, obs: Any, state: Any = None, info: dict[str, Any] | None = None) -> tuple[torch.Tensor, Any]:
+        action, hidden = self.preprocess(obs, state)
+        return self.max_action * torch.tanh(self.last(action)), hidden
 
 
 class ContinuousActorProbabilistic(ModuleWithVectorOutput):
